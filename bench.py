@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — DiT denoising steps/sec (2048 primitive tokens, CFG x2) on N B200s, plus VAE decode ms.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): image-conditioned DDIM, CFG 6, 2048 tokens x 1370 context tokens, fp16, ONE
 sample per GPU.  A *step* is one `forward_with_cfg` (two sequences) + the sampler update.  Synthetic weights of the
@@ -16,6 +16,11 @@ shipped architecture and synthetic inputs of the shipped shapes (no checkpoints 
   roofline tcgen05 GEMM kernel family: algorithmic FLOPs of the GEMMs in a step / their summed device time, measured
            live with per-launch CUDA events (a separate profiled pass of the same steps); peak from MEASURED_PEAKS.json.
   cpu_baseline / --impl reference: the staged reference modules (oracle/_ref; the oracle port only if they are absent), fp32, host cores.
+
+  --dump-outputs DIR  after the timed steps, rank 0 writes what the last timed step returned to its caller as DIR/<name>.npy (float32):
+           model_output (forward_with_cfg), sample and pred_xstart (the sampler update); with --config 5, sample and recon_param of the
+           last generation.  Weights and inputs are seeded, so two builds run with the same arguments can be compared output for output.
+           Past 64 MB in all, each array is replaced by the same share of its elements, flattened, at sorted positions drawn from a fixed seed.
 """
 from __future__ import annotations
 
@@ -32,6 +37,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "DiT steps/sec (2048 prim tokens, CFG x2)"
 UNIT = "steps/s"
@@ -67,6 +73,22 @@ def f_step_executed() -> dict:
 
 
 F_VAE = 4.593e12   # SURVEY.md §8a a14: 2242.8 MFLOP per primitive x 2048
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(dirname: str, tensors: dict) -> None:
+    """--dump-outputs: each tensor as <dirname>/<name>.npy in float32; over DUMP_BYTES in all, a fixed seeded sample of each."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in tensors.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_BYTES - 1024 * len(arrays)                     # room for the .npy headers
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if total > budget:
+            keep = a.size * budget // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+    print(f"[bench] wrote {', '.join(arrays)} to {dirname}" + (" (sampled)" if total > budget else ""), file=sys.stderr, flush=True)
 
 
 def load_peaks():
@@ -224,7 +246,7 @@ def run_reference(args):
         return
     # one untimed step pages the 3.6 GB of fp32 parameters in and spins the thread pool up; then whole steps are timed
     n_warm = min(max(args.warmup, 0), 1)
-    r = cpu_steps(n_warm=n_warm, n_timed=max(args.steps, 1), budget_s=float(os.environ.get("TPX_REF_BUDGET_S", "170")))
+    r = cpu_steps(n_warm=n_warm, n_timed=args.steps, budget_s=float("inf"))      # exactly --steps timed steps
     n = len(r["per_step_s"])
     sample = f"{n} whole steps timed ({r['what']}); requested --steps {args.steps} --warmup {args.warmup}, {n_warm} untimed warm-up step(s), no extrapolation"
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": n, "warmup": n_warm,
@@ -293,12 +315,16 @@ def run_ours(args):
         if hoist:
             model.set_timesteps(tmap, force=True)
 
+    last = {}                                                   # what the latest step returned to its caller (--dump-outputs)
+
     def one_step(x, y, i, use_table=True):
         t = t_all[i % nT].expand(BS).contiguous()
         out = model.forward_with_cfg(x, t, y, cfg_scale=CFG_SCALE, precision_dtype=torch.float16, enable_amp=True,
                                      t_host=tmap[i % nT] if (hoist and use_table) else None)
         noise = torch.randn_like(x)
-        return diffusion._step(True, x, out, i % nT, 0.0, False, noise)["sample"]
+        step = diffusion._step(True, x, out, i % nT, 0.0, False, noise)
+        last.update(step, model_output=out)
+        return step["sample"]
 
     _note("model ready")
     # ---- device-resident timing ("value") ----
@@ -324,6 +350,7 @@ def run_ours(args):
         launches = lib.tpx_launch_count() - l0
         ms_dev = e0.elapsed_time(e1)
         clock_info = clocks.stop(mark) if clocks else None
+        outputs = dict(last)                                    # the last timed step's results (the later legs take new steps)
 
         _note(f"value leg done: {ms_dev:.2f} ms")
         # the same K steps with every forward recomputing the timestep MLP + adaLN pass (what the table replaces): in-run A/B, not a headline
@@ -446,6 +473,8 @@ def run_ours(args):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
     peaks = load_peaks()
     # Both measured peaks are reported.  The timed loop is a fraction of a second at ~1.95 GHz (not the power-throttled regime the
@@ -552,7 +581,9 @@ def run_config5(args):
     def generation():          # host buffers in, host buffers out: this IS the end-to-end path
         y = y_host.to(dev, non_blocking=True)
         x = noise.to(dev, non_blocking=True)
-        out_host.copy_(pipe(y, x)["recon_param"], non_blocking=True)
+        res = pipe(y, x)
+        out_host.copy_(res["recon_param"], non_blocking=True)
+        return res
 
     for _ in range(W):
         generation()
@@ -564,12 +595,14 @@ def run_config5(args):
     barrier()
     e0.record()
     for _ in range(K):
-        generation()
+        res = generation()
     e1.record()
     barrier()
     launches = lib.tpx_launch_count() - l0
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
     clock_info = clocks.stop(mark) if clocks else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sample": res["sample"], "recon_param": out_host})
     # split of one generation: the DDIM loop alone vs decode + glue
     y, x = y_host.to(dev), noise.to(dev)
     d = pipe.make_diffusion()
@@ -621,7 +654,12 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 5], help="2 = BASELINE configs[1] (the headline: DiT steps/s); 5 = configs[4] "
                     "(end-to-end DDIM-100 + VAE decode, 4 samples per GPU, samples/s; here --steps counts whole generations)")
     ap.add_argument("--ddim", type=int, default=100, help="DDIM steps of --config 5")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (float32, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path; the reference arm has other weights and inputs")
     # The contract is ONE JSON line on stdout.  Native libraries write there too (NCCL prints its version banner to fd 1 when
     # NCCL_DEBUG=VERSION is set on the box), so fd 1 is pointed at stderr for the whole run and the result line goes to the
     # saved descriptor.

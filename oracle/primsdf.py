@@ -10,8 +10,20 @@ Dense O(points x prims) torch math, for small problem sizes.
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 import torch.nn.functional as F
+
+
+def fixture_scene(seed: int, K: int = 96, S: int = 8, n: int = 4000, dim_feat: int = 6):
+    """The seeded scene of tests/golden/primsdf.npz (tests/golden/make_golden.py), rebuilt instead of stored: numpy
+    RandomState(seed) draws, in this order, srt [K,4] (scale in [0.05, 0.25], centre in [-0.8, 0.8]^3), feat [K, dim_feat*S^3]
+    standard normal and n points in [-1, 1]^3.  -> (srt, feat, pts), float32 arrays."""
+    rs = np.random.RandomState(seed)
+    srt = np.concatenate([rs.uniform(0.05, 0.25, size=(K, 1)), rs.uniform(-0.8, 0.8, size=(K, 3))], axis=1).astype(np.float32)
+    feat = rs.standard_normal(size=(K, dim_feat * S ** 3)).astype(np.float32)
+    pts = rs.uniform(-1, 1, size=(n, 3)).astype(np.float32)
+    return srt, feat, pts
 
 
 def local_grid(S: int) -> torch.Tensor:

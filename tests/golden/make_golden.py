@@ -95,8 +95,8 @@ def main():
         for h in hooks:
             h.remove()
         cfg_out = model.forward_with_cfg(x, t, y, cfg_scale=6.0)
-        if tag == "dit_full1":        # keep the fixture small: every 8th token of forward, the full CFG output in fp16-exact halves
-            fwd = fwd[:, ::8]
+        if tag == "dit_full1":        # keep the fixture under 1 MB: every 8th token of both outputs
+            fwd, cfg_out = fwd[:, ::8], cfg_out[:, ::8]
         np.savez_compressed(os.path.join(OUT, tag + ".npz"), cfg=json.dumps(cfg), M=M, seed=seed, t=t.numpy(),
                             forward=fwd.numpy(), forward_with_cfg=cfg_out.numpy(),
                             blocks=np.stack([b.numpy() for b in blocks]) if tag == "dit_tiny" else np.zeros(0),
@@ -173,23 +173,20 @@ def main():
     # ---- PrimSDF point query (SURVEY §8f-1): the reference class, with `trimesh` (imported but unused on this path) stubbed
     sys.modules.setdefault("trimesh", types.ModuleType("trimesh"))
     from models.primsdf import PrimSDF              # noqa: E402
-    rs = np.random.RandomState(1104)
-    K, S = 96, 8
-    srt = np.concatenate([rs.uniform(0.05, 0.25, size=(K, 1)), rs.uniform(-0.8, 0.8, size=(K, 3))], axis=1).astype(np.float32)
-    feat = rs.standard_normal(size=(K, 6 * S ** 3)).astype(np.float32)
-    pts = rs.uniform(-1, 1, size=(4000, 3)).astype(np.float32)
+    sys.path.insert(0, ROOT)
+    import oracle                                                            # noqa: E402  (scene / weight synthesis shared with the tests)
+    srt, feat, pts = oracle.primsdf.fixture_scene(1104)
+    K, S = srt.shape[0], 8
     m = PrimSDF(num_prims=K, dim_feat=6, prim_shape=S).eval()
     m.srt_param.data = torch.from_numpy(srt)
     m.feat_param.data = torch.from_numpy(feat)
     preds = m(torch.from_numpy(pts))
     covered = (m.prim_weight(torch.from_numpy(pts)).sum(1) > 0).numpy()
-    np.savez_compressed(os.path.join(OUT, "primsdf.npz"), srt=srt, feat=feat, pts=pts, covered=covered,
+    np.savez_compressed(os.path.join(OUT, "primsdf.npz"), seed=1104, covered=covered,
                         sdf=preds["sdf"].numpy(), tex=preds["tex"].numpy(), mat=preds["mat"].numpy())
     print("primsdf", int(covered.sum()), "of", len(pts), "points covered")
 
     # ---- DINOv2 ViT-B/14-reg encoder (SURVEY §8f-2): the reference wrapper, random weights instead of the hub download --------
-    sys.path.insert(0, ROOT)
-    import oracle                                                            # noqa: E402  (weight synthesis shared with the tests)
     from models.conditioner.image_dinov2 import Dinov2Wrapper               # noqa: E402
     import models.conditioner.dinov2.hub.backbones as bb                     # noqa: E402
     Dinov2Wrapper._build_dinov2 = staticmethod(lambda model_name, modulation_dim=None, pretrained=True:

@@ -40,6 +40,40 @@ def test_product_arm_has_no_cpu_path():
     assert p.stdout.strip() == ""
 
 
+def test_bad_arguments_are_refused_before_any_work():
+    for args in (("--steps", "0"), ("--impl", "reference", "--dump-outputs", "out")):
+        p = _run(*args, timeout=120)
+        assert p.returncode == 2 and p.stdout.strip() == "", args
+
+
+def test_dump_outputs_writes_float32_and_samples_past_the_limit(tmp_path):
+    import importlib.util
+
+    import numpy as np
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    flag = sys.dont_write_bytecode
+    try:
+        spec.loader.exec_module(bench)
+    finally:
+        sys.dont_write_bytecode = flag
+    small = {"sample": torch.randn(1, 2048, 68), "model_output": torch.randn(1, 2048, 136).half()}
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    for k, v in small.items():
+        a = np.load(tmp_path / "small" / f"{k}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, v.float().numpy())
+    big = {"recon_param": torch.randn(4, 2048, 3076), "sample": torch.randn(4, 2048, 68)}      # --config 5: 103 MB
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), big)
+    written = sum(os.path.getsize(tmp_path / "a" / f"{k}.npy") for k in big)
+    assert 0.99 * bench.DUMP_BYTES < written <= bench.DUMP_BYTES
+    for k in big:
+        a, b = (np.load(tmp_path / d / f"{k}.npy") for d in ("a", "b"))
+        assert a.dtype == np.float32 and np.array_equal(a, b)                                    # the same sample every run
+    assert np.isin(a, big["sample"].numpy()).all()
+
+
 def test_reference_arm_under_torchrun_prints_once():
     """N > 1: rank 0 alone measures and prints; the other rank exits 0 without work."""
     import socket

@@ -22,13 +22,14 @@ def _module(srt, feat, K, S=8):
 
 def test_matches_reference_fixture(golden_dir):
     fx = np.load(os.path.join(golden_dir, "primsdf.npz"))
-    m = _module(fx["srt"], fx["feat"], fx["srt"].shape[0])
-    out = m(torch.from_numpy(fx["pts"]).cuda())
+    srt, feat, pts = oracle.primsdf.fixture_scene(int(fx["seed"]))
+    m = _module(srt, feat, srt.shape[0])
+    out = m(torch.from_numpy(pts).cuda())
     for k in ("sdf", "tex", "mat"):
         np.testing.assert_allclose(out[k].cpu().numpy(), fx[k], err_msg=k, **TOL)
     cov = torch.from_numpy(fx["covered"])
     m.train()
-    tr = m(torch.from_numpy(fx["pts"]).cuda())
+    tr = m(torch.from_numpy(pts).cuda())
     assert float(tr["sdf"].cpu()[~cov].abs().max()) == 0.0
     np.testing.assert_allclose(tr["sdf"].cpu().numpy()[fx["covered"]], fx["sdf"][fx["covered"]], **TOL)
 
