@@ -26,6 +26,10 @@ class VaeConfig(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("latent_channels", "out_channels", "ch_mid", "ch_out", "attn_heads")]
 
 
+class VaeEncoderConfig(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("in_channels", "latent_channels", "ch0", "ch1", "attn_heads")]
+
+
 class SamplerCoefs(C.Structure):
     _fields_ = [(n, C.c_float) for n in ("sqrt_ab", "sqrt_1mab", "sqrt_recip_ab", "sqrt_recipm1_ab", "c_x0", "c_eps", "sigma", "nonzero",
                                          "coef1", "coef2", "min_log", "max_log")] + [("clip", C.c_int32)]
@@ -61,6 +65,14 @@ SIGNATURES = {
     "tpx_vae_finalize": (_i, [_vp, _vp]),
     "tpx_vae_workspace_bytes": (_sz, [_vp, _i]),
     "tpx_vae_decode": (_i, [_vp, _vp, _i, _vp, _i, _i, _vp, _sz, _vp]),
+    "tpx_vae_encoder_create": (_i, [C.POINTER(VaeEncoderConfig), C.POINTER(_vp)]),
+    "tpx_vae_encoder_destroy": (None, [_vp]),
+    "tpx_vae_encoder_set_weight": (_i, [_vp, C.c_char_p, _vp, _i, C.POINTER(_i64), _i, _vp]),
+    "tpx_vae_encoder_finalize": (_i, [_vp, _vp]),
+    "tpx_vae_encoder_workspace_bytes": (_sz, [_vp, _i]),
+    "tpx_vae_encode": (_i, [_vp, _vp, _i, _vp, _i, _i, _vp, _sz, _vp]),
+    "tpx_vae_encode_stage": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _sz, _vp]),
+    "tpx_vae_posterior": (_i, [_vp, _i, _i64, _i64, _i, _vp, _vp, _vp, _vp]),
     "tpx_linear": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _i, _vp]),
     "tpx_linear_gated": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _i, _i, _i, _i, _i, _vp]),
     "tpx_linear_heads": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _i, _vp]),
@@ -78,6 +90,7 @@ SIGNATURES = {
     "tpx_primsdf_query_grid": (_i, [_vp, _vp, _vp, _vp, _sz, _i64, _i, _i, _i, _i, _vp, _vp]),
     "tpx_groupnorm_silu": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _vp, _vp]),
     "tpx_conv3d_k3": (_i, [_vp, _vp, _vp, _vp, _f, _vp, _i, _i, _i, _i, _vp]),
+    "tpx_conv3d_k3_s2": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
 }
 
 

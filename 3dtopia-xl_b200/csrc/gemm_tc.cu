@@ -134,19 +134,25 @@ static int map_2d(const void* ptr, long long rows, long long K, long long ld, in
     return TPX_OK;
 }
 
-// 5-D: channels-last volume [P, S, S, S, C] fp16; box = 128 voxel rows x bk channels
-static int map_conv(const void* ptr, long long P, int S, int C, int bk, CUtensorMap* out) {
-    MapKey key{ptr, P, S, C, 0, bk, 5 * 16 + 2};
+// 5-D: channels-last volume [P, S, S, S, C] fp16; box = 128 voxel rows x bk channels.  stride2: S = 8 input traversed with element
+// stride 2 in x / y / z, so the 8^3 x 2-primitive box lands as 4^3 x 2 = 128 rows (AMODE_CONV3_S2)
+static int map_conv(const void* ptr, long long P, int S, int C, int bk, CUtensorMap* out, bool stride2 = false) {
+    MapKey key{ptr, P, S, C, stride2 ? 2 : 0, bk, 5 * 16 + 2};
     std::lock_guard<std::mutex> lk(g_maps_mu);
     auto it = g_maps.find(key);
     if (it != g_maps.end()) { *out = it->second; return TPX_OK; }
     EncodeTiledFn enc = encode_fn();
     TPX_CHECK(enc != nullptr, TPX_ERR_CUDA, "cuTensorMapEncodeTiled unavailable (no driver?)");
     TPX_CHECK(S == 4 || S == 8, TPX_ERR_SHAPE, "conv volume edge must be 4 or 8, got %d", S);
+    TPX_CHECK(!stride2 || S == 8, TPX_ERR_SHAPE, "stride-2 conv input edge must be 8, got %d", S);
     cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)S, (cuuint64_t)S, (cuuint64_t)S, (cuuint64_t)P};
     cuuint64_t gstr[4] = {(cuuint64_t)C * 2, (cuuint64_t)S * C * 2, (cuuint64_t)S * S * C * 2, (cuuint64_t)S * S * S * C * 2};
     cuuint32_t box[5] = {(cuuint32_t)bk, (cuuint32_t)S, (cuuint32_t)S, (cuuint32_t)(S == 4 ? 4 : 2), (cuuint32_t)(S == 4 ? 2 : 1)};
     cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+    if (stride2) {   // ceil(8 / 2) = 4 elements per spatial dimension land in shared memory
+        box[1] = box[2] = box[3] = 8; box[4] = 2;
+        estr[1] = estr[2] = estr[3] = 2;
+    }
     CUtensorMap m;
     CUresult r = enc(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<void*>(ptr), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      swizzle_for(bk), CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -310,25 +316,29 @@ int launch_gemm_2cta(const GemmProblem& p, cudaStream_t stream) {
 int launch_gemm(const GemmProblem& p, cudaStream_t stream) {
     TPX_CHECK(p.M > 0 && p.N > 0 && p.K > 0, TPX_ERR_SHAPE, "gemm: empty problem %d x %d x %d", p.M, p.N, p.K);
     TPX_CHECK(p.N % 8 == 0 && p.K % 8 == 0, TPX_ERR_SHAPE, "gemm: N (%d) and K (%d) must be multiples of 8", p.N, p.K);
-    const int bk = (p.a_mode == AMODE_CONV3 && p.conv_C == 32) ? 32 : 64;
-    ProfScope prof(p.a_mode == AMODE_CONV3 ? PROF_CONV_GEMM : PROF_GEMM, stream);
+    const bool conv = p.a_mode == AMODE_CONV3 || p.a_mode == AMODE_CONV3_S2;
+    const int bk = (conv && p.conv_C == 32) ? 32 : 64;
+    ProfScope prof(conv ? PROF_CONV_GEMM : PROF_GEMM, stream);
     GemmArgs a = p.args;
     a.M = p.M;
     a.N = p.N;
     a.num_kb = (p.K + bk - 1) / bk;
     a.dbg = g_gemm_dbg;
     a.conv_S = p.conv_S;
-    a.chunks_per_tap = p.a_mode == AMODE_CONV3 ? p.conv_C / bk : 1;
+    a.chunks_per_tap = conv ? p.conv_C / bk : 1;
     CUtensorMap ta, tb;
     int rc;
     if (p.a_mode == AMODE_LINEAR) {
         rc = map_2d(p.A, p.M, p.K, p.lda, 128, bk, &ta);
     } else {
         TPX_CHECK(p.conv_C % bk == 0 && p.K == 27 * p.conv_C, TPX_ERR_SHAPE, "conv gemm: K (%d) must be 27*C (%d)", p.K, p.conv_C);
-        const int s3 = p.conv_S * p.conv_S * p.conv_S;
-        TPX_CHECK(p.M % s3 == 0, TPX_ERR_SHAPE, "conv gemm: M (%d) must be P*S^3", p.M);
-        rc = map_conv(p.A, p.M / s3, p.conv_S, p.conv_C, bk, &ta);
+        const bool s2 = p.a_mode == AMODE_CONV3_S2;
+        const int so = s2 ? p.conv_S / 2 : p.conv_S, s3 = so * so * so;   // output voxels per primitive
+        TPX_CHECK(p.M % s3 == 0, TPX_ERR_SHAPE, "conv gemm: M (%d) must be P*S_out^3", p.M);
+        rc = map_conv(p.A, p.M / s3, p.conv_S, p.conv_C, bk, &ta, s2);
     }
+    TPX_CHECK(p.epi != EPI_NCDHW_MIX || (a.mix != nullptr && a.n_valid >= 1 && a.n_valid <= 4 && a.n_valid <= p.N), TPX_ERR_ARG,
+              "gemm: channel-mix epilogue needs its weights and 1..4 valid channels (got %d)", a.n_valid);
     if (rc != TPX_OK) return rc;
     rc = map_2d(p.W, p.N, p.K, p.K, p.BN, bk, &tb);
     if (rc != TPX_OK) return rc;
@@ -363,6 +373,10 @@ int launch_gemm(const GemmProblem& p, cudaStream_t stream) {
     TPX_CASE(32, 32, AMODE_CONV3, EPI_STORE)
     TPX_CASE(32, 32, AMODE_CONV3, EPI_RESID_SCALE)
     TPX_CASE(16, 32, AMODE_CONV3, EPI_NCDHW)
+    // VAE encoder
+    TPX_CASE(32, 32, AMODE_CONV3_S2, EPI_STORE)     // down_blocks.0.downsample 32 -> 32, 8^3 -> 4^3
+    TPX_CASE(256, 32, AMODE_CONV3, EPI_STORE)       // down_blocks.1.nets.0.conv1 32 -> 256 at 4^3
+    TPX_CASE(16, 64, AMODE_CONV3, EPI_NCDHW_MIX)    // conv_out 256 -> 2 (N padded to 16) with quant_conv folded in
 #undef TPX_CASE
     set_error("gemm: no kernel instantiated for BN=%d BK=%d amode=%d epi=%d", p.BN, bk, p.a_mode, p.epi);
     return TPX_ERR_SHAPE;

@@ -10,6 +10,9 @@
 // A-operand modes: AMODE_LINEAR (2-D tensor map over a row-major [M,K] fp16 matrix) and AMODE_CONV3 (5-D tensor
 // map over a channels-last [P,S,S,S,C] fp16 volume: the 27 taps of a 3x3x3 / pad 1 convolution are 27 shifted
 // box loads, the halo comes from TMA out-of-bounds zero fill — implicit GEMM with no im2col buffer).
+// AMODE_CONV3_S2 is the stride-2 version over an 8^3 input (the encoder's downsample, vae3d_dib.py:168): the tensor
+// map traverses x / y / z with element stride 2, so one box of 8^3 voxels delivers the 4^3 input voxels a tap reads
+// for two primitives (128 rows); the tap offset is the box start (dx-1, dy-1, dz-1), the pad-1 halo the zero fill.
 #pragma once
 #include "tpx_common.cuh"
 
@@ -23,8 +26,9 @@ enum GemmEpiMode : int {
     EPI_RESID_SCALE = 4, // out0 = h( (acc + bias + resid[row*ldo+col]) * alpha )
     EPI_CONVT2 = 5,      // k2s2 transposed conv scatter: col=(abc,co), row=(p,z,y,x)@4^3 -> channels-last 8^3
     EPI_NCDHW = 6,       // out[(p*Cout+co)*S3 + vox] = acc + bias   (fp32 or fp16 out, co < n_valid)
+    EPI_NCDHW_MIX = 7,   // out[(p*n_valid+j)*S3 + vox] = sum_c mix[j,c] * h(acc_c + bias_c) + mix_bias[j]   (a 1x1 conv folded in)
 };
-enum GemmAMode : int { AMODE_LINEAR = 0, AMODE_CONV3 = 1 };
+enum GemmAMode : int { AMODE_LINEAR = 0, AMODE_CONV3 = 1, AMODE_CONV3_S2 = 2 };
 
 struct GemmArgs {
     int M, N, num_kb;
@@ -50,6 +54,7 @@ struct GemmArgs {
     int pdl_trigger;  // 2-CTA kernel: 1 = griddepcontrol.launch_dependents after the prologue (launched with the PDL attribute)
     int heads_tma;    // EPI_HEADS: 1 = outputs leave as 24-column bulk tensor stores (launcher checked the geometry, padding is pre-zeroed)
     long long* dbg;   // timeline probe (tpx_debug_gemm_timeline): 16 int64 per CTA, nullptr in the product path
+    const __half* mix;   // EPI_NCDHW_MIX: [n_valid, n_valid] channel-mix weight followed by its [n_valid] bias (n_valid <= 4)
 };
 
 template <int BN, int BK>
@@ -263,6 +268,26 @@ __device__ __forceinline__ void epi_chunk(const GemmArgs& g, const float* __rest
                 const size_t off = (static_cast<size_t>(p) * g.n_valid + co) * g.S3 + vox;
                 if (g.out32 != nullptr) g.out32[off] = v[i];
                 else g.out0[off] = __float2half_rn(v[i]);
+            }
+        }
+    } else if constexpr (EPI == EPI_NCDHW_MIX) {
+        // the convolution's n_valid channels of this row round to fp16 (one rounding per layer), then the 1x1 mix runs in fp32 on them
+        const int p = row / g.S3, vox = row - p * g.S3;
+        const int nv = g.n_valid;
+        float hc[4];
+#pragma unroll
+        for (int c = 0; c < 4; ++c) hc[c] = h2f_round(v[c]);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (j >= nv) break;
+            float s = __half2float(g.mix[nv * nv + j]);
+#pragma unroll
+            for (int c = 0; c < 4; ++c)
+                if (c < nv) s = fmaf(__half2float(g.mix[j * nv + c]), hc[c], s);
+            if (row_ok) {
+                const size_t off = (static_cast<size_t>(p) * nv + j) * g.S3 + vox;
+                if (g.out32 != nullptr) g.out32[off] = s;
+                else g.out0[off] = __float2half_rn(s);
             }
         }
     }
@@ -554,7 +579,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     } else {
                         const int tap = kb / g.chunks_per_tap, chunk = kb - tap * g.chunks_per_tap;
                         const int dz = tap / 9, dy = (tap / 3) % 3, dx = tap % 3;
-                        if (g.conv_S == 4) {  // 128 rows = 2 primitives x 4^3 voxels
+                        if (AMODE == AMODE_CONV3_S2 || g.conv_S == 4) {  // 128 rows = 2 primitives x 4^3 (output) voxels
                             tma_load_5d(sa, &tmA, &full_bar[stage], chunk * BK, dx - 1, dy - 1, dz - 1, m_blk * 2);
                         } else {              // S == 8: 128 rows = 2 z-slices of one primitive
                             tma_load_5d(sa, &tmA, &full_bar[stage], chunk * BK, dx - 1, dy - 1, (m_blk & 3) * 2 + dz - 1, m_blk >> 2);

@@ -57,6 +57,9 @@ int launch_vae_conv_in(const void* z, int z_dtype, const __half* w_pq, const __h
                        __half* out, cudaStream_t st);
 int launch_groupnorm_silu(const __half* x, const __half* gamma, const __half* beta, int P, int S3, int C, int groups, float eps, int apply_silu,
                           __half* out, cudaStream_t st);
+int launch_vae_pack_input(const void* x, int dtype, int P, int Cin, int CP, __half* out, cudaStream_t st);
+int launch_vae_posterior(const void* params, int dtype, long long B, long long half, int deterministic, void* logvar, void* stdv, void* var,
+                         cudaStream_t st);
 
 // primsdf.cu : PrimSDF point query; out [n,6] = (sdf, rgb clipped, rough/metal clipped)
 int launch_primsdf_query(const float* x, const float* srt, const float* feat, long long n, int K, int S, int dim_feat, int inference, float* out,

@@ -400,19 +400,97 @@ int launch_groupnorm_silu(const __half* x, const __half* gamma, const __half* be
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// VAE encoder input: x [P, Cin, 8, 8, 8] NCDHW (fp32 / fp16) -> channels-last fp16 [P, 512, CP], channels Cin..CP-1 zero, so the
+// 6-channel conv_in runs on the 32-channel halo convolution (its packed weights have zero columns there).  One thread per voxel:
+// the Cin loads are coalesced across the warp's voxels, the CP-channel row leaves as 16-byte stores.
+// ---------------------------------------------------------------------------------------------------------
+template <typename T, int CP>
+__global__ void __launch_bounds__(256) vae_pack_input_kernel(const T* __restrict__ x, int P, int Cin, __half* __restrict__ out) {
+    const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= static_cast<long long>(P) * 512) return;
+    const long long p = i >> 9;
+    const int vox = static_cast<int>(i & 511);
+    const T* src = x + p * Cin * 512 + vox;
+    uint4* dst = reinterpret_cast<uint4*>(out + i * CP);
+#pragma unroll
+    for (int o = 0; o < CP / 8; ++o) {
+        Pack8 v;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            const int c = o * 8 + k;
+            v.h[k] = c < Cin ? __float2half_rn(static_cast<float>(src[static_cast<long long>(c) * 512])) : __float2half_rn(0.f);
+        }
+        dst[o] = v.u;
+    }
+}
+
+int launch_vae_pack_input(const void* x, int dtype, int P, int Cin, int CP, __half* out, cudaStream_t st) {
+    TPX_CHECK(CP == 32 && Cin >= 1 && Cin <= CP, TPX_ERR_SHAPE, "vae_pack_input: %d input channels into %d unsupported", Cin, CP);
+    if (P <= 0) return TPX_OK;
+    ProfScope prof(PROF_VAE_MISC, st);
+    const unsigned grid = static_cast<unsigned>((static_cast<long long>(P) * 512 + 255) / 256);
+    if (dtype == TPX_DTYPE_F32) vae_pack_input_kernel<float, 32><<<grid, 256, 0, st>>>(static_cast<const float*>(x), P, Cin, out);
+    else if (dtype == TPX_DTYPE_F16) vae_pack_input_kernel<__half, 32><<<grid, 256, 0, st>>>(static_cast<const __half*>(x), P, Cin, out);
+    else { set_error("vae_pack_input: unsupported input dtype %d", dtype); return TPX_ERR_ARG; }
+    TPX_LAUNCH_CHECK();
+    return TPX_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// DiagonalGaussianDistribution fields (vae3d_dib.py:51-60) in the parameters' dtype, the reference's operation order:
+// logvar = clamp(params[:, half:], -30, 20); std = exp(0.5 * logvar); var = exp(logvar) — each op rounded to T as torch does;
+// deterministic: std = var = 0.  params [B, 2 * half] (the mean is the first half, a view on the host side).
+// ---------------------------------------------------------------------------------------------------------
+template <typename T>
+__global__ void vae_posterior_kernel(const T* __restrict__ params, long long B, long long half, int deterministic, T* __restrict__ logvar,
+                                     T* __restrict__ stdv, T* __restrict__ var) {
+    const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i >= B * half) return;
+    const long long b = i / half, j = i - b * half;
+    const float lv = fminf(fmaxf(static_cast<float>(params[b * 2 * half + half + j]), -30.0f), 20.0f);
+    logvar[i] = static_cast<T>(lv);
+    if (deterministic) {
+        stdv[i] = static_cast<T>(0.0f);
+        var[i] = static_cast<T>(0.0f);
+    } else {
+        const float hl = static_cast<float>(static_cast<T>(0.5f * lv));
+        stdv[i] = static_cast<T>(expf(hl));
+        var[i] = static_cast<T>(expf(lv));
+    }
+}
+
+int launch_vae_posterior(const void* params, int dtype, long long B, long long half, int deterministic, void* logvar, void* stdv, void* var,
+                         cudaStream_t st) {
+    if (B * half == 0) return TPX_OK;
+    ProfScope prof(PROF_VAE_MISC, st);
+    const unsigned grid = static_cast<unsigned>((B * half + 255) / 256);
+    if (dtype == TPX_DTYPE_F32)
+        vae_posterior_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(params), B, half, deterministic, static_cast<float*>(logvar),
+                                                          static_cast<float*>(stdv), static_cast<float*>(var));
+    else if (dtype == TPX_DTYPE_F16)
+        vae_posterior_kernel<__half><<<grid, 256, 0, st>>>(static_cast<const __half*>(params), B, half, deterministic, static_cast<__half*>(logvar),
+                                                           static_cast<__half*>(stdv), static_cast<__half*>(var));
+    else { set_error("vae_posterior: unsupported dtype %d", dtype); return TPX_ERR_ARG; }
+    TPX_LAUNCH_CHECK();
+    return TPX_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // weight repacks (run once at load time)
 // ---------------------------------------------------------------------------------------------------------
-// Conv3d weight [Cout,Cin,3,3,3] -> [CoutPad, 27*Cin] with k = tap*Cin + ci, tap = (kz*3+ky)*3+kx.
+// Conv3d weight [Cout,Cin,3,3,3] -> [CoutPad, 27*CinP] with k = tap*CinP + ci, tap = (kz*3+ky)*3+kx; columns ci >= Cin are zero
+// (CinP > Cin: the encoder's conv_in, whose input is zero-padded to CinP channels).
 // transposed != 0: source is a ConvTranspose3d(k3,s1,p1) weight [Cin,Cout,3,3,3]; the equivalent correlation
 // kernel is w'[co,ci,kz,ky,kx] = w[ci,co,2-kz,2-ky,2-kx]  (vae3d_dib.py:367).
 template <typename T>
-__global__ void pack_conv3_kernel(const T* __restrict__ src, __half* __restrict__ dst, int Cout, int Cin, int transposed) {
+__global__ void pack_conv3_kernel(const T* __restrict__ src, __half* __restrict__ dst, int Cout, int Cin, int CinP, int transposed) {
     const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-    const long long n = static_cast<long long>(Cout) * 27 * Cin;
+    const long long n = static_cast<long long>(Cout) * 27 * CinP;
     if (i >= n) return;
-    const int co = static_cast<int>(i / (27 * Cin));
-    const int r = static_cast<int>(i - static_cast<long long>(co) * 27 * Cin);
-    const int tap = r / Cin, ci = r - tap * Cin;
+    const int co = static_cast<int>(i / (27 * CinP));
+    const int r = static_cast<int>(i - static_cast<long long>(co) * 27 * CinP);
+    const int tap = r / CinP, ci = r - tap * CinP;
+    if (ci >= Cin) { dst[i] = __float2half_rn(0.f); return; }
     size_t s;
     if (!transposed) s = (static_cast<size_t>(co) * Cin + ci) * 27 + tap;
     else s = (static_cast<size_t>(ci) * Cout + co) * 27 + (26 - tap);
@@ -429,11 +507,12 @@ __global__ void pack_convt2_kernel(const T* __restrict__ src, __half* __restrict
     dst[i] = __float2half_rn(static_cast<float>(src[(static_cast<size_t>(ci) * Cout + co) * 8 + abc]));
 }
 
-int launch_pack_conv3(const void* src, int dtype, __half* dst, int Cout, int Cin, int transposed, cudaStream_t st) {
-    const long long n = static_cast<long long>(Cout) * 27 * Cin;
+int launch_pack_conv3(const void* src, int dtype, __half* dst, int Cout, int Cin, int transposed, cudaStream_t st, int CinP) {
+    if (CinP < Cin) CinP = Cin;
+    const long long n = static_cast<long long>(Cout) * 27 * CinP;
     const unsigned grid = static_cast<unsigned>((n + 255) / 256);
-    if (dtype == TPX_DTYPE_F32) pack_conv3_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(src), dst, Cout, Cin, transposed);
-    else if (dtype == TPX_DTYPE_F16) pack_conv3_kernel<__half><<<grid, 256, 0, st>>>(static_cast<const __half*>(src), dst, Cout, Cin, transposed);
+    if (dtype == TPX_DTYPE_F32) pack_conv3_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(src), dst, Cout, Cin, CinP, transposed);
+    else if (dtype == TPX_DTYPE_F16) pack_conv3_kernel<__half><<<grid, 256, 0, st>>>(static_cast<const __half*>(src), dst, Cout, Cin, CinP, transposed);
     else { set_error("pack_conv3: unsupported dtype %d", dtype); return TPX_ERR_ARG; }
     TPX_LAUNCH_CHECK();
     return TPX_OK;

@@ -3,7 +3,7 @@
 Parameter NAMES and SHAPES are the reference's checkpoint contract (SURVEY.md §8b):
   DiT  — /root/reference/models/dit_crossattn.py:111-156 (module tree), attention.py:37-39,83-87,
          utils.py:31-36,85-92
-  VAE  — /root/reference/models/vae3d_dib.py:330-367 (Decoder), :429 (post_quant_conv)
+  VAE  — /root/reference/models/vae3d_dib.py:330-367 (Decoder), :429 (post_quant_conv), :270-307 (Encoder), :428 (quant_conv)
 Values are drawn from numpy's frozen ``RandomState`` stream so the golden fixtures under
 tests/golden/ can be regenerated bit-identically on any box; ``device_state_dict`` draws on the GPU
 instead (fast path for full-size benchmarks, values need not match anything).
@@ -88,6 +88,33 @@ def vae_decoder_shapes(latent_channels=1, out_channels=6, up_channels=(256, 32),
     s[d + "norm_out.weight"], s[d + "norm_out.bias"] = (cout,), (cout,)
     s[d + "conv_out.weight"], s[d + "conv_out.bias"] = (cout, out_channels, 3, 3, 3), (out_channels,)
     s["post_quant_conv.weight"], s["post_quant_conv.bias"] = (latent_channels,) * 2 + (1, 1, 1), (latent_channels,)
+    return s
+
+
+def vae_encoder_shapes(in_channels=1, latent_channels=1, down_channels=(32, 256), mid_attention=True,
+                       layers_per_block=2, **_) -> "OrderedDict[str, Tuple[int, ...]]":
+    """encoder.* / quant_conv.* keys of VAE (vae3d_dib.py:270-307 Encoder, :428 quant_conv)."""
+    s: "OrderedDict[str, Tuple[int, ...]]" = OrderedDict()
+    e = "encoder."
+    c0 = down_channels[0]
+    s[e + "conv_in.weight"], s[e + "conv_in.bias"] = (c0, in_channels, 3, 3, 3), (c0,)
+    cout = c0
+    for i, ch in enumerate(down_channels):
+        cin, cout = cout, ch
+        for j in range(layers_per_block):
+            _resnet_shapes(s, f"{e}down_blocks.{i}.nets.{j}.", cin if j == 0 else cout, cout)
+        if i != len(down_channels) - 1:
+            s[f"{e}down_blocks.{i}.downsample.weight"], s[f"{e}down_blocks.{i}.downsample.bias"] = (cout, cout, 3, 3, 3), (cout,)
+    _resnet_shapes(s, e + "mid_block.nets.0.", cout, cout)
+    _resnet_shapes(s, e + "mid_block.nets.1.", cout, cout)
+    if mid_attention:
+        a = e + "mid_block.attns.0."
+        s[a + "norm.weight"], s[a + "norm.bias"] = (cout,), (cout,)
+        s[a + "attn.qkv.weight"] = (3 * cout, cout)
+        s[a + "attn.proj.weight"], s[a + "attn.proj.bias"] = (cout, cout), (cout,)
+    s[e + "norm_out.weight"], s[e + "norm_out.bias"] = (cout,), (cout,)
+    s[e + "conv_out.weight"], s[e + "conv_out.bias"] = (2 * latent_channels, cout, 3, 3, 3), (2 * latent_channels,)
+    s["quant_conv.weight"], s["quant_conv.bias"] = (2 * latent_channels,) * 2 + (1, 1, 1), (2 * latent_channels,)
     return s
 
 

@@ -159,6 +159,39 @@ size_t tpx_vae_workspace_bytes(const tpx_vae* h, int P);
 int tpx_vae_decode(tpx_vae* h, const void* z_dev, int z_dtype, void* out_dev, int out_dtype, int P, void* ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * VAE encoder — models/vae3d_dib.py:270-327 (Encoder), :428-435 (quant_conv, VAE.encode), :50-60 (DiagonalGaussianDistribution).
+ * A handle of its own: the decoder handle, its workspace and its key contract are independent of it.
+ * ---------------------------------------------------------------------------------------------------------- */
+typedef struct tpx_vae_encoder tpx_vae_encoder;
+typedef struct tpx_vae_encoder_config {
+    int32_t in_channels;     /* 6 (1..16) */
+    int32_t latent_channels; /* 1 */
+    int32_t ch0;             /* down_channels[0] = 32 */
+    int32_t ch1;             /* down_channels[1] = 256 */
+    int32_t attn_heads;      /* 8 (head dim 32) */
+} tpx_vae_encoder_config;
+/* Encoder.__init__ + quant_conv (vae3d_dib.py:284-307, 428) for the released layout only; anything else -> TPX_ERR_SHAPE. */
+int tpx_vae_encoder_create(const tpx_vae_encoder_config* cfg, tpx_vae_encoder** out);
+void tpx_vae_encoder_destroy(tpx_vae_encoder* h);
+/* load_state_dict(sd['model_state_dict']): encoder.* / quant_conv.* keys are consumed (fp32 or fp16 sources), decoder.* /
+ * post_quant_conv.* keys are accepted and ignored (return 1). */
+int tpx_vae_encoder_set_weight(tpx_vae_encoder* h, const char* ref_key, const void* dev_ptr, int dtype, const int64_t* shape, int ndim, void* stream);
+int tpx_vae_encoder_finalize(tpx_vae_encoder* h, void* stream);
+size_t tpx_vae_encoder_workspace_bytes(const tpx_vae_encoder* h, int P);
+/* VAE.encode up to the posterior's parameters (vae3d_dib.py:431-433): x device [P,in_channels,8,8,8] (dtype x_dtype) ->
+ * params device [P,2*latent,4,4,4] (dtype params_dtype) = quant_conv(Encoder(x)). */
+int tpx_vae_encode(tpx_vae_encoder* h, const void* x_dev, int x_dtype, void* params_dev, int params_dtype, int P, void* ws, size_t ws_bytes,
+                   void* stream);
+/* The same schedule stopped after stage 1 conv_in, 2 down_blocks.0 (after the stride-2 conv), 3 down_blocks.1 or 4 mid_block
+ * (vae3d_dib.py:313-320): out_f16 device channels-last [P,S,S,S,C] of that activation.  Parity aid. */
+int tpx_vae_encode_stage(tpx_vae_encoder* h, const void* x_dev, int x_dtype, int P, int stage, void* out_f16, void* ws, size_t ws_bytes, void* stream);
+/* DiagonalGaussianDistribution.__init__ (vae3d_dib.py:51-60): params device [batch, 2*half_elems] (dtype fp32 / fp16; the mean is
+ * its first half per batch row) -> logvar = clamp(second half, -30, 20), std = exp(0.5 logvar), var = exp(logvar), each device
+ * [batch, half_elems] in the same dtype; deterministic != 0 gives std = var = 0. */
+int tpx_vae_posterior(const void* params_dev, int dtype, int64_t batch, int64_t half_elems, int deterministic, void* logvar_dev, void* std_dev,
+                      void* var_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * Per-kernel entry points (unit parity tests; each is one launch of one hot-path kernel)
  * ---------------------------------------------------------------------------------------------------------- */
 /* out[M,N] fp16 = act(A[M,K] W[N,K]^T + bias) ; act: 0 none (optionally * post_scale, re-rounded), 1 GELU-tanh.  tile_n: 0 = auto. */
@@ -199,6 +232,9 @@ int tpx_groupnorm_silu(const void* x_f16, const void* gamma_f16, const void* bet
  * W_f16 is [Cout, 27*C] with k = tap*C + c, tap = (kz*3+ky)*3+kx;  out [P,S,S,S,Cout] fp16 = (conv + bias (+ resid)) * alpha. */
 int tpx_conv3d_k3(const void* x_f16, const void* W_f16, const void* bias_f16, const void* resid_f16, float alpha, void* out_f16, int P, int S, int C,
                   int Cout, void* stream);
+/* Stride-2 3x3x3 / pad 1 convolution (vae3d_dib.py:168, DownBlock.downsample): x [P,8,8,8,C] -> out [P,4,4,4,Cout] fp16, W as above
+ * (C = Cout = 32). */
+int tpx_conv3d_k3_s2(const void* x_f16, const void* W_f16, const void* bias_f16, void* out_f16, int P, int C, int Cout, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * PrimSDF point query — models/primsdf.py:52-109 (PrimSDF.forward = prim_weight + grid_sample_feat), the consumer of

@@ -5,7 +5,7 @@ T=${1:-600}
 mkdir -p gpurun_out
 nvidia-smi --query-gpu=name,clocks.sm,clocks.max.sm,memory.total --format=csv > gpurun_out/gpu.txt 2>&1
 rc_all=0
-for f in tests/test_gpu_gemm.py tests/test_gpu_elementwise.py tests/test_gpu_attention.py tests/test_gpu_dit.py tests/test_gpu_sampler.py tests/test_gpu_vae.py tests/test_gpu_primsdf.py tests/test_gpu_pipeline.py tests/test_gpu_raymarch.py tests/test_gpu_ref_fp16.py tests/test_gpu_zz_extra.py; do
+for f in tests/test_gpu_gemm.py tests/test_gpu_elementwise.py tests/test_gpu_attention.py tests/test_gpu_dit.py tests/test_gpu_sampler.py tests/test_gpu_vae.py tests/test_gpu_vae_encode.py tests/test_gpu_primsdf.py tests/test_gpu_pipeline.py tests/test_gpu_raymarch.py tests/test_gpu_ref_fp16.py tests/test_gpu_zz_extra.py; do
   n=$(basename $f .py)
   timeout $T python -m pytest $f -q -m gpu --timeout 300 --no-header -p no:cacheprovider -s > gpurun_out/$n.log 2>&1
   rc=$?
